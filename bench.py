@@ -20,6 +20,8 @@ and the process exits non-zero on a mismatch.
 
   --impl reference   times the CPU oracle instead (the reference is Go; no Go toolchain exists here or on the
                      GPU box, so the "reference arm" is the restatement in oracle/, all host threads).
+  --dump-outputs DIR writes the results of every action of the last timed step as DIR/<action>_<field>.npy (float64),
+                     so that two builds run with the same arguments (same seeded inputs) can be compared array by array.
 """
 from __future__ import annotations
 
@@ -53,6 +55,38 @@ def measured_peak_gbs():
         except Exception:
             pass
     return 6650.0, "fallback"
+
+
+DUMP_LIMIT_BYTES = 60_000_000  # below 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, results):
+    """Writes the results of one step, [(action, abi.Result)] in run order, as out_dir/<action>_<field>.npy in float64
+    (exact for the int32 fields).  Every array's last axis runs over tasks, visits, queues or nodes.  When the whole
+    exceeds DUMP_LIMIT_BYTES, every array keeps the same fixed-seed sample of its last axis (arrays of equal length keep
+    the same positions) and <action>_<field>_index.npy lists the kept positions."""
+    names = [a for a, _ in results]
+    arrays = {}
+    for i, (action, r) in enumerate(results):
+        tag = action if names.count(action) == 1 else f"{action}{i}"
+        fields = {"task_node": r.task_node, "task_status": r.task_status,
+                  "visit_job": r.visits[:, 0], "visit_outcome": r.visits[:, 1],
+                  "queue_fair_share": r.queue_fair_share, "queue_allocated": r.queue_allocated,
+                  "queue_allocated_non_preemptible": r.queue_allocated_non_preemptible,
+                  "queue_request": r.queue_request, "total_resource": r.total_resource,
+                  "node_idle": r.node_idle, "node_releasing": r.node_releasing,
+                  "pods_placed_evicted": [r.pods_placed, r.pods_evicted]}
+        arrays.update({f"{tag}_{k}": np.asarray(v, dtype=np.float64) for k, v in fields.items()})
+    total = sum(a.nbytes for a in arrays.values())
+    keep = 1.0 if total <= DUMP_LIMIT_BYTES else DUMP_LIMIT_BYTES / (2 * total)  # 2: room for the index arrays
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        n = a.shape[-1]
+        if keep < 1.0 and n > 1:
+            idx = np.sort(np.random.default_rng(0).choice(n, max(1, int(n * keep)), replace=False))
+            a = a[..., idx]
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -131,14 +165,17 @@ def run_reference(args, snap, workload, actions=("allocate",), engine_kw=None):
     for i in range(args.warmup + args.steps):
         o.load(sample)
         t0 = time.perf_counter()
-        moved = 0
+        moved, outputs = 0, []
         for a in s_actions:
             res = o.run(a)
+            outputs.append((a, res))
             moved += res.pods_placed + res.pods_evicted
         dt = time.perf_counter() - t0
         if i >= args.warmup:
             times.append(dt)
             placed += moved
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     total = sum(times)
     value = placed / total
     line = {
@@ -170,7 +207,11 @@ def main():
     ap.add_argument("--snapshot", default=None,
                     help="time a recorded cluster instead of a synthetic config: a zip of the reference's snapshot "
                          "plugin (kai_scheduler_b200/snapshot_io.py); actions and plugin arguments come from the file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the results of every action of the last timed step to DIR/<action>_<field>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     rank, world, local = dist_env()
 
@@ -245,14 +286,20 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def one_step():
-        """returns (device_ms, e2e_s, pods, stats)"""
+    def one_step(keep=None):
+        """returns (device_ms, e2e_s, pods, stats); `keep` (a list) receives a copy of every action's result, made off the
+        e2e clock (the engine's result buffers only live until the next run)"""
         t0 = time.perf_counter()
+        copy_s = 0.0
         eng.load_c(c_snap, snap.n_res)       # H2D of the whole snapshot + open-session kernels
         dev, moved, launches_, alg_, act_ = 0.0, 0, 0, 0, 0.0
         one_step.evicted, one_step.decisions = 0, 0
         for a in actions:
             r = eng.run(a, copy=False)       # action kernel + D2H of the results
+            if keep is not None:
+                tc = time.perf_counter()
+                keep.append((a, abi.Result.from_c(r, snap.n_res)))
+                copy_s += time.perf_counter() - tc
             st = eng.stats()
             dev += st.action_ms
             moved += int(r.pods_placed) + int(r.pods_evicted)
@@ -261,7 +308,7 @@ def main():
             launches_ = int(st.kernel_launches)
             alg_ += int(st.algorithmic_bytes)
             act_ += st.action_ms
-        e2e = time.perf_counter() - t0
+        e2e = time.perf_counter() - t0 - copy_s
         st.kernel_launches, st.algorithmic_bytes, st.action_ms = launches_, alg_, act_
         return st.open_session_ms + dev, e2e, moved, st, r
 
@@ -274,8 +321,9 @@ def main():
     phase_ms = {"upload": 0.0, "open_session": 0.0, "action": 0.0, "download": 0.0}
     t_wall0 = time.perf_counter()
     decisions = evicted_e = 0
-    for _ in range(args.steps):
-        d, e, p, st, r = one_step()
+    outputs = []
+    for i in range(args.steps):
+        d, e, p, st, r = one_step(outputs if args.dump_outputs and rank == 0 and i == args.steps - 1 else None)
         decisions, evicted_e = one_step.decisions, one_step.evicted
         dev_ms += d
         e2e_s += e
@@ -291,6 +339,8 @@ def main():
     barrier()
     wall = time.perf_counter() - t_wall0
     clocks = sampler.stop()
+    if outputs:
+        dump_outputs(args.dump_outputs, outputs)
     last = abi.Result.from_c(r, snap.n_res)  # outcome of the last timed step (copied out of the engine's buffers)
     ranks_agree = True
     if world > 1:  # every rank runs the same sequencer over its node stripe: the bindings must be identical everywhere
