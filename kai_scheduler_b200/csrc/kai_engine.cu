@@ -1109,6 +1109,12 @@ int kai_engine_run(kai_engine *e, kai_action action, kai_result *out) {
     hb.topm = p.topm;
     hb.prof = getenv("KAI_PROFILE") != nullptr;
     for (int i = 0; i < 8; i++) hb.t_sec[i] = 0;
+    for (int i = 0; i < 4; i++) hb.t_pop_split[i] = 0;
+    {  // job order of the allocate action: "keyed" (default; used when the snapshot allows it) or "replica"
+      const char *jo = getenv("KAI_JOB_ORDER");
+      hb.keyed_order_allowed = !(jo && strcmp(jo, "replica") == 0);
+      hb.keyed_order_used = false;
+    }
     hb.h_list = e->cfg.shard_count > 1 ? e->shm_base + (size_t)2 * 2 * kMaxGrid * kSlotWords : e->h_list;
     hb.n_list_scanners = e->cfg.shard_count * (e->grid - 1);
     hb.launch_mode = launch_mode;
@@ -1369,6 +1375,16 @@ int kai_engine_run(kai_engine *e, kai_action action, kai_result *out) {
     if (host_mode)
       fprintf(stderr, "[kai] host sequencer rdtsc Mcycles: pop %.2f admit %.2f place(+sweeps) %.2f finish %.2f loop %.2f\n",
               e->hb.t_sec[0] / 1e6, e->hb.t_sec[1] / 1e6, e->hb.t_sec[2] / 1e6, e->hb.t_sec[3] / 1e6, e->hb.t_sec[4] / 1e6);
+    if (host_mode && !solver_action) {
+      if (e->hb.keyed_order_used)
+        fprintf(stderr, "[kai] job order: keyed; eligibility check %.3f Mcycles, tree build %.3f Mcycles\n", e->hb.t_sec[5] / 1e6,
+                e->hb.t_sec[6] / 1e6);
+      else
+        fprintf(stderr, "[kai] job order: replica (%s, queue %d); eligibility check %.3f Mcycles, tree build %.3f Mcycles; pop Mcycles: fix root %.2f fix children %.2f keys %.2f leaf pop + handle_pop %.2f\n",
+                e->hb.korder.reason, e->hb.korder.reason_queue,
+                e->hb.t_sec[5] / 1e6, e->hb.t_sec[6] / 1e6, e->hb.t_pop_split[0] / 1e6, e->hb.t_pop_split[1] / 1e6,
+                e->hb.t_pop_split[2] / 1e6, e->hb.t_pop_split[3] / 1e6);
+    }
     if (host_mode && c[45] > 0)
       fprintf(stderr, "[kai] %s: %lld cycles per list (%lld lists): load %lld, sort %lld, prefix + payload %lld, stream out %lld, fence + header %lld\n",
               e->merge_cluster ? "k_merge_cluster" : "k_merge", c[44] / c[45], c[45], c[39] / c[45], c[46] / c[45], c[31] / c[45], c[47] / c[45], c[43] / c[45]);
@@ -1401,6 +1417,7 @@ int kai_engine_run(kai_engine *e, kai_action action, kai_result *out) {
     return e->fail(KAI_ERR_CUDA, m2);
   }
   if (c[6] == 2) return e->fail(KAI_ERR_UNSUPPORTED, "topology: more preferred-level domains than the score table holds (kDomBuckets)");
+  if (c[6] == 3) return e->fail(KAI_ERR_STATE, "keyed job order: a popped job still has pending tasks (KAI_JOB_ORDER=replica runs the replica order)");
   if (c[6] != 0) return e->fail(KAI_ERR_CUDA, "device sequencer overflow (statement log)");
   return download(e, out, c[0], c[3], c[4]);
 }

@@ -20,6 +20,7 @@
 #include <vector>
 
 #include "kai_action.cuh"
+#include "kai_job_order.cuh"
 #include "kai_seq.cuh"
 #include "kai_topology.cuh"
 
@@ -83,7 +84,13 @@ struct HostBackend {
   }
 
   bool prof = false;
-  unsigned long long t_sec[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // rdtsc: pop, admit, place (incl. sweeps), finish, loop
+  // rdtsc: pop, admit, place (incl. sweeps), finish, loop, job-order eligibility check, job-order tree build
+  unsigned long long t_sec[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  unsigned long long t_pop_split[4] = {0, 0, 0, 0};  // replica pop: fix root, fix children, keys, leaf pop + handle_pop
+  // ---- job order of run_allocate: the keyed order (kai_job_order.cuh) when the snapshot allows it, else the replica ----
+  bool keyed_order_allowed = true;  // false: KAI_JOB_ORDER=replica
+  bool keyed_order_used = false;    // what the last run_allocate did
+  KeyedJobOrder korder;
   int trace_kind[64];
   unsigned int trace_seq[64];
   int trace_nd[64];
@@ -711,7 +718,6 @@ struct HostBackend {
     const DevSnap &s = *seq.s;
     double t_begin = now();
     t_exchange = 0;
-    seq_init_job_order(seq);
     unsigned long long tk = prof ? __builtin_ia32_rdtsc() : 0;
     auto lap = [&](int i) {
       if (!prof) return;
@@ -719,9 +725,20 @@ struct HostBackend {
       t_sec[i] += t - tk;
       tk = t;
     };
+    korder.reason = "KAI_JOB_ORDER=replica";
+    korder.reason_queue = -1;
+    const bool keyed = keyed_order_allowed && korder.check(seq);
+    keyed_order_used = keyed;
+    lap(5);
+    if (keyed)
+      korder.build(seq);
+    else
+      seq_init_job_order(seq);
+    lap(6);
+    seq.pop_split = prof && !keyed ? t_pop_split : nullptr;
     for (;;) {
       lap(4);
-      int job = pop_next_job(seq);
+      int job = keyed ? korder.pop(seq) : pop_next_job(seq);
       lap(0);
       if (job < 0 || failed) break;
       seq.n_ops = 0;
@@ -771,7 +788,12 @@ struct HostBackend {
         if (should_pipeline_job(seq, job)) stmt_convert_all_allocated_to_pipelined(seq, job);
         stmt_commit(seq);
         record_visit(seq, job, 1);
-        if (has_tasks_to_allocate(seq, job)) push_job(seq, job);
+        if (has_tasks_to_allocate(seq, job)) {
+          if (keyed)
+            seq.error = 3;  // KeyedJobOrder::check rules this out; the keyed heaps cannot take the job back
+          else
+            push_job(seq, job);
+        }
       } else {
         stmt_rollback(seq, 0);
         record_visit(seq, job, 0);
@@ -784,6 +806,7 @@ struct HostBackend {
       lap(3);
       if (seq.error || failed) break;
     }
+    seq.pop_split = nullptr;
     publish(DK_DONE);  // carries the last node deltas; the scanners write their tiles back and exit
     t_total = now() - t_begin;
   }

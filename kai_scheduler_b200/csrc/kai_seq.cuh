@@ -242,6 +242,10 @@ struct Seq {  // sequencer state (lane 0 of warp 0 of CTA 0)
   int error;
   long long t_pop, t_prep, t_scan, t_xchg, t_apply, t_finish, t_init;  // clock64 phase totals (thread 0)
   long long t_key, n_key, t_tta, t_heap;
+  // host-sequenced mode, KAI_PROFILE only: rdtsc split of pop_next_job (null = off; never set on the device)
+  unsigned long long *pop_split;  // [4]: fix root heap, fix child heaps, key recomputation, leaf pop + handle_pop
+  unsigned long long pop_mark;
+  long long pop_key_mark;
 };
 
 KAI_HD inline double &q_alloc(Seq &q, int r, int qi) { return q.rp.q_alloc[(size_t)r * q.s->Q + qi]; }
@@ -716,10 +720,32 @@ KAI_HD int best_job(Seq &q, int qi) {  // :283-292 getBestJobFromNode
 
 // queue_order.go:19-73 on cached per-node keys.  A key is recomputed when the queue's Allocated or its
 // best pending job changed since it was last used (invalidate_chain / queue_allocate).
+// clock of the key-recomputation counter: clock64 on the device, rdtsc on the host while the pop is profiled
+KAI_HD inline long long key_clock(const Seq &q) {
+#ifdef __CUDA_ARCH__
+  return clock64();
+#else
+  return q.pop_split ? (long long)__builtin_ia32_rdtsc() : 0;
+#endif
+}
+// host pop profile: charge the time since the last mark to section i, less the key recomputations inside it
+KAI_HD inline void pop_lap(Seq &q, int i) {
+#ifndef __CUDA_ARCH__
+  if (!q.pop_split) return;
+  const unsigned long long t = __builtin_ia32_rdtsc();
+  const long long keys = q.t_key - q.pop_key_mark;
+  if (i >= 0) {
+    q.pop_split[i] += (t - q.pop_mark) - (unsigned long long)keys;
+    q.pop_split[2] += (unsigned long long)keys;
+  }
+  q.pop_mark = t;
+  q.pop_key_mark = q.t_key;
+#endif
+}
 KAI_HD const QKey &queue_key(Seq &q, int qi) {
   QKey &k = q.rp.qkey[qi];
   if (k.valid) return k;
-  long long tkk = kclock();
+  long long tkk = key_clock(q);
   q.n_key++;
   const DevSnap &s = *q.s;
   const double *req = job_init_resource(q, best_job(q, qi));
@@ -748,7 +774,7 @@ KAI_HD const QKey &queue_key(Seq &q, int qi) {
   k.w0 = ((unsigned long long)(over ? 1 : 0) << 44) | ((unsigned long long)(starved ? 0 : 1) << 43) |
          (((unsigned long long)(0x80000000LL - (long long)k.priority) & 0x1ffffffffull) << 10) | ((unsigned long long)(viol ? 1 : 0) << 9);
   k.valid = 1;
-  q.t_key += kclock() - tkk;
+  q.t_key += key_clock(q) - tkk;
   return k;
 }
 KAI_HD bool node_less(Seq &q, int l, int r) {  // :256-278 buildNodeOrderFn (pending order)
@@ -892,9 +918,12 @@ KAI_HD void handle_pop(Seq &q, int qi) {  // :219-243
 }
 KAI_HD int pop_next_job(Seq &q) {  // :61-88
   if (q.root_len == 0) return -1;
+  pop_lap(q, -1);
   int ni = get_next_node(q, q.rp.root_heap, q.root_len, -1);
+  pop_lap(q, 0);
   while (ni >= 0 && !qn_is_leaf(q, ni))
     ni = get_next_node(q, q.rp.child_heap + kldg(&q.s->q_child_begin[ni]), q.rp.child_len[ni], ni);
+  pop_lap(q, 1);
   if (ni < 0) return -1;
   int job = leaf_pop(q, ni);
   {  // warm L1 for the next pops of this queue
@@ -907,6 +936,7 @@ KAI_HD int pop_next_job(Seq &q) {  // :61-88
   }
   invalidate_chain(q, ni);
   handle_pop(q, ni);
+  pop_lap(q, 3);
   return job;
 }
 
